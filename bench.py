@@ -9,6 +9,7 @@ work ``OneFormAssembler.assemble`` does in steady state (SURVEY.md section 3.2).
 
     python bench.py --gpus 1 --steps 10 --warmup 3
     python bench.py --impl reference            # CPU restatement on the host cores
+    python bench.py --dump-outputs DIR          # also write the last step's result to DIR/y.npy
 
 Prints ONE JSON line (see the key list in DESIGN.md section "Measurement").
 """
@@ -28,6 +29,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 METRIC = "assembled DoFs/sec (Poisson CG3, 256^3 hex, 1-form/action)"
+DUMP_ROWS = 1 << 22          # --dump-outputs: at most 32 MiB of float64 over all ranks
 
 
 def parse():
@@ -48,7 +50,14 @@ def parse():
                          "no local->global reduce (SURVEY.md 8e option ii); 'sum' = the reference's owned cells + "
                          "ghost-sum reduce")
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the owned rows of the assembled vector of the last step "
+                         "to DIR/y.npy (DIR/y_rank<R>.npy with several GPUs), float64; above %d rows in all, "
+                         "the rows at fixed seeded indices" % DUMP_ROWS)
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 # ------------------------------------------------------------------ clocks
@@ -138,6 +147,19 @@ def make_problem(args, rank, world, pinned):
     y = op2.Dat(dnodes, pinned=pinned)
     X = op2.Dat(op2.DataSet(vnodes, 3), mesh.coordinates)
     return part, mesh, V, cells, m0, m1, x, y, X
+
+
+def dump_outputs(out_dir, y, nowned, rank, world):
+    """--dump-outputs: the owned rows of ``y`` as a caller reads them (``y.data_ro``); beyond
+    DUMP_ROWS / world rows per rank, the rows at sorted indices drawn with a fixed seed, so that
+    two builds run with the same arguments write the same rows."""
+    rows = y.data_ro[:nowned]
+    k = DUMP_ROWS // world
+    if nowned > k:
+        rows = rows[np.unique(np.random.default_rng(0).integers(0, nowned, k))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "y.npy" if world == 1 else f"y_rank{rank}.npy"),
+            np.asarray(rows, dtype=np.float64))
 
 
 def algorithmic_bytes(V, mesh):
@@ -424,6 +446,8 @@ def main():
         step()
     _lib.check(L.fdb_timer_stop(tm, C.byref(ms)))
     barrier()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, y, ndof_owned, rank, world)
     total_ms = maxreduce(ms.value)
     launches = L.fdb_launch_count() - launches0
     # kernel-only duration (CUDA events around the global kernel alone, same

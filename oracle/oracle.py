@@ -7,18 +7,19 @@ Two builds of ``oracle.c``:
 
 * ``_build/liboracle.so`` -- portable ``-march=x86-64-v3``; built by
   ``__graft_entry__.build()`` in the CPU container and shipped to the GPU box;
-* ``_build/liboracle_native.so`` -- ``-march=native`` as PyOP2's JIT uses
-  (reference pyop2/compilation.py:341-363), compiled on first use ON THE BOX
-  THAT RUNS IT (the build container's CPU differs from the GPU box's host).
+* ``-march=native`` as PyOP2's JIT uses (reference pyop2/compilation.py:341-363),
+  compiled on first use in each process ON THE MACHINE THAT RUNS IT (the build
+  machine's CPU may differ from the GPU host's), in a temporary directory that
+  is removed once the library is loaded, so the source tree may be read-only.
   Used for timing when gcc is available, else falls back to the portable one.
 """
 from __future__ import annotations
 
 import ctypes
-import hashlib
 import os
-import platform
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -34,7 +35,7 @@ c_lp = ctypes.POINTER(ctypes.c_int64)
 
 
 def _compile(out, march):
-    os.makedirs(BUILD, exist_ok=True)
+    os.makedirs(os.path.dirname(out), exist_ok=True)
     cmd = ["gcc", *BASE_FLAGS, f"-march={march}", "-o", out, *SRC, "-lm"]
     subprocess.run(cmd, check=True, cwd=HERE, capture_output=True)
     return out
@@ -49,22 +50,12 @@ def build(force=False):
     return out
 
 
-def _cpu_tag():
+def _load_native():
+    tmp = tempfile.mkdtemp(prefix="fdb_oracle_")
     try:
-        with open("/proc/cpuinfo") as f:
-            txt = f.read()
-        model = [l for l in txt.splitlines() if l.startswith(("model name", "flags"))][:2]
-    except OSError:
-        model = [platform.processor()]
-    src = b"".join(open(s, "rb").read() for s in SRC + [os.path.join(HERE, "hex_kernels.inc")])
-    return hashlib.sha1(("".join(model)).encode() + src).hexdigest()[:12]
-
-
-def build_native():
-    out = os.path.join(BUILD, f"liboracle_native_{_cpu_tag()}.so")
-    if not os.path.exists(out):
-        _compile(out, "native")
-    return out
+        return ctypes.CDLL(_compile(os.path.join(tmp, "liboracle_native.so"), "native"))
+    finally:
+        shutil.rmtree(tmp, ignore_errors=True)
 
 
 class _W(ctypes.Structure):
@@ -80,15 +71,15 @@ def lib(native=False):
     key = bool(native)
     if key in _lib:
         return _lib[key]
-    path = None
+    L = None
     if native:
         try:
-            path = build_native()
+            L, path = _load_native(), "liboracle_native.so"
         except Exception:
-            path = None
-    if path is None:
+            pass
+    if L is None:
         path = build()
-    L = ctypes.CDLL(path)
+        L = ctypes.CDLL(path)
     L.orc_build_sparsity.restype = ctypes.c_int64
     L.orc_vec_dot.restype = ctypes.c_double
     _lib[key] = L
