@@ -917,7 +917,7 @@ int fdb_jit_call(fdb_kernel_s *k, const fdb_call_args *a)
         p.layer_hi = nl = j->lay_max;
         p.ncl = 1;
     } else if (pl.extruded) {
-        // layer extents by iteration region (pyop2/codegen/builder.py:779-800); layers[] counts
+        // layer extents by iteration region (pyop2/codegen/builder.py:790-812); layers[] counts
         // NODE layers, so cells are [layers[0], layers[1]-1)
         const int cs = a->layers[0], ce = a->layers[1] - 1;
         p.bottom = cs;
@@ -925,7 +925,10 @@ int fdb_jit_call(fdb_kernel_s *k, const fdb_call_args *a)
         switch (pl.region) {
         case FDB_REGION_ON_BOTTOM: p.layer_lo = cs; p.layer_hi = cs + 1; break;
         case FDB_REGION_ON_TOP: p.layer_lo = ce - 1; p.layer_hi = ce; break;
-        case FDB_REGION_ON_INTERIOR_FACETS: p.layer_lo = cs; p.layer_hi = ce - 1; break;
+        // a periodic column also has the facet between its top and bottom cells: the
+        // last layer's "above" cell wraps round to the bottom through the % p.ncl of the
+        // map index (tests/test_wrapper_semantics.py, periodic ON_INTERIOR_FACETS cases)
+        case FDB_REGION_ON_INTERIOR_FACETS: p.layer_lo = cs; p.layer_hi = pl.periodic ? ce : ce - 1; break;
         default: p.layer_lo = cs; p.layer_hi = ce; break;
         }
         nl = p.layer_hi - p.layer_lo;

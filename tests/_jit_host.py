@@ -90,10 +90,17 @@ def tallest(layers, region):
     return int(max(cells.max(), 0))
 
 
-def run(spec, start, end, args, maps, layers=None, subset=None, region="ALL"):
+def extents(cs, ce, region, periodic=False):
+    """Layer extent of the launch grid for constant layers, cells ``[cs, ce)`` (fdb_jit_call):
+    a periodic column has ``ce - cs`` interior horizontal facets, the last one wrapping round."""
+    return {"ALL": (cs, ce), "ON_BOTTOM": (cs, cs + 1), "ON_TOP": (ce - 1, ce),
+            "ON_INTERIOR_FACETS": (cs, ce if periodic else ce - 1)}[region]
+
+
+def run(spec, start, end, args, maps, layers=None, subset=None, region="ALL", periodic=False):
     """Execute the generated wrapper on host arrays.  ``args``: one entry per
     kernel argument -- numpy array (Dat / Global) or HostCSR (Mat); ``maps``: the
-    int32 map arrays in slot order."""
+    int32 map arrays in slot order; ``periodic``: the set is periodically extruded."""
     fn, _ = build(spec.source(), spec.kernel.name)
     p = WrapParams()
     p.start, p.end = start, end
@@ -108,8 +115,7 @@ def run(spec, start, end, args, maps, layers=None, subset=None, region="ALL"):
         cs, ce = int(layers[0]), int(layers[1]) - 1
         p.bottom = cs
         p.ncl = max(ce - cs, 1)
-        lo, hi = {"ALL": (cs, ce), "ON_BOTTOM": (cs, cs + 1), "ON_TOP": (ce - 1, ce),
-                  "ON_INTERIOR_FACETS": (cs, ce - 1)}[region]
+        lo, hi = extents(cs, ce, region, periodic)
         p.layer_lo, p.layer_hi = lo, hi
         nl = max(hi - lo, 0)
     keep = []

@@ -359,7 +359,7 @@ class MockEngine:
         self._next += 1
         self.kernels[self._next] = dict(kind="jit", fn=fn, keep=keep, args=args, extruded=d.extruded,
                                         subset=d.subset, region=d.iteration_region, name=name,
-                                        varlay=d.variable_layers)
+                                        varlay=d.variable_layers, periodic=d.extruded_periodic)
         _obj(out).value = self._next
         return 0
 
@@ -390,7 +390,8 @@ class MockEngine:
             cs, ce = a.layers[0], a.layers[1] - 1
             p.bottom = cs
             p.ncl = max(ce - cs, 1)
-            lo, hi = {0: (cs, ce), 1: (cs, cs + 1), 2: (ce - 1, ce), 3: (cs, ce - 1)}[k["region"]]
+            region = ("ALL", "ON_BOTTOM", "ON_TOP", "ON_INTERIOR_FACETS")[k["region"]]
+            lo, hi = jh.extents(cs, ce, region, bool(k["periodic"]))
             p.layer_lo, p.layer_hi = lo, hi
             nl = max(hi - lo, 0)
         p.subset = _addr(a.subset) or None

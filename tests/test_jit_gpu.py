@@ -461,6 +461,31 @@ def test_periodic_extrusion_on_device(engine, oracle):
     assert np.abs(z.data_ro).max() < 1e-12
 
 
+def test_periodic_interior_horizontal_facets_on_device(engine):
+    """dS_h on periodically extruded columns: a column of nz cells has nz horizontal interior
+    facets, the last one joining its top cell to its bottom cell (pyop2/codegen/builder.py:800-805).
+    Counted three ways: a Global INC (nz per column), the sum of the layer numbers into a Dat
+    indexed by the column (0 + ... + nz-1), and a cell Dat through a periodic map that every
+    facet adds 1 to below and 10 to above (11 in every cell, the bottom cell's 10 coming from
+    the wrap-around facet)."""
+    from firedrake_b200 import codegen
+    ncol, nz = 37, 6
+    cols = op2.ExtrudedSet(op2.Set(ncol), nz + 1, extruded_periodic=True)
+    cells = op2.Set(ncol * nz)
+    cmap = op2.Map(cols, cells, 1, np.arange(ncol) * nz, offset=[1])     # cell l of column c: c*nz + l
+    k = op2.Kernel("static void k(double *g, double *s, double *c, int layer) "
+                   "{ g[0] += 1.0; s[0] += layer; c[0] += 1.0; c[1] += 10.0; }", "k")
+    for location in ("device", "host"):
+        g = op2.Global(1, 0.0)
+        s = op2.Dat(op2.DataSet(cols, 1))
+        c = op2.Dat(cells)
+        codegen.par_loop(k, cols, g(op2.INC), s(op2.INC), c(op2.INC, cmap), iteration_region="ON_INTERIOR_FACETS",
+                         pass_layer_arg=True, location=location)
+        assert g.data_ro[0] == ncol * nz, location
+        assert (s.data_ro == nz * (nz - 1) // 2).all(), location
+        assert (c.data_ro == 11.0).all(), location
+
+
 def test_mixed_dat_parloop_and_vector_operations(engine):
     """op2.MixedDat through op2.par_loop on the device and in host-pointer mode (one local tensor
     for the kernel, one arglist pointer per block: pyop2/parloop.py:203-212), plus the block-wise
