@@ -299,8 +299,11 @@ int fdb_kernel_create(const fdb_kernel_desc *d, fdb_kernel_t *out)
         set_error("fdb_kernel_create: rank must be 1 or 2");
         return 1;
     }
-    if (d->cdim < 1 || d->cdim > 3) {
-        set_error("fdb_kernel_create: cdim %d outside 1..3", d->cdim);
+    // 2-forms assemble the scalar matrix and add it into the block diagonals (A (x) I_cdim), so any
+    // block size the blocked store / SpMV kernels of mat.cu instantiate (1..4) is fine there
+    const int max_cdim = d->rank == 2 ? 4 : 3;
+    if (d->cdim < 1 || d->cdim > max_cdim) {
+        set_error("fdb_kernel_create: cdim %d outside 1..%d", d->cdim, max_cdim);
         return 1;
     }
     if (d->cell == FDB_CELL_HEX_EXTRUDED && (!d->offset0 || !d->offset1)) {

@@ -1010,6 +1010,12 @@ class Mat:
             sp = self.sparsity
             rmap = sp.mono_map if rmap is sp.maps[0] else self._mono_map_of(rmap)
             cmap = sp.mono_map if cmap is sp.maps[0] else self._mono_map_of(cmap)
+        elif getattr(self, "sparsity", None) is not None and \
+                not (rmap is self.sparsity.maps[0] and cmap is self.sparsity.maps[0]):
+            # pyop2/types/mat.py:439-441.  The scatter finds an entry's position from the sparsity's
+            # map (the rank table is per column of that map), so another map over the same sets
+            # would add its values at wrong positions without any error
+            raise MapValueError("Path maps not in sparsity maps")
         a = LegacyArg(self, access, rmap)
         a.cmap = cmap
         a.lgmaps = lgmaps

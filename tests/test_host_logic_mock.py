@@ -165,3 +165,27 @@ def test_solve_front_end_host_logic(mock, pc):
 
 def test_variable_coefficient_host_logic(mock, oracle):
     tj.test_variable_coefficient_form(mock, oracle)
+
+
+def test_mat_path_maps_must_be_the_sparsity_maps(mock):
+    """``mat(op2.INC, (rmap, cmap))`` with maps other than the sparsity's raises MapValueError
+    (pyop2/types/mat.py:439-441), even when they have the same iteration and target sets: the scatter
+    locates entries through the sparsity's map, so another map's values would land at wrong positions."""
+    from firedrake_b200 import op2
+    import test_matrix_gpu as tm
+    mesh = tm.ExtrudedHexMesh(3, 2, 3, warp=0.05)
+    V, cells, nodes, m0, m1, X = tm.setup(mesh, 2)
+    mat = op2.Mat(op2.Sparsity((nodes, nodes), [(m0, m0, None)]))
+    perm = np.random.default_rng(0).permutation(mesh.num_base_cells)
+    m2 = op2.Map(cells, nodes, V.arity, V.cell_node_map[perm], offset=V.offset)
+    m0_copy = op2.Map(cells, nodes, V.arity, V.cell_node_map.copy(), offset=V.offset)
+    for path in [(m2, m2), (m0, m2), (m2, m0), (m0_copy, m0_copy)]:
+        with pytest.raises(op2.MapValueError):
+            mat(op2.INC, path)
+    k = op2.Kernel("helmholtz", degree=2, rank=2)
+    op2.par_loop(k, cells, mat(op2.INC, (m0, m0)), X(op2.READ, m1))
+    # blocked matrices take the same check
+    bmat = op2.Mat(op2.Sparsity((op2.DataSet(nodes, 2), op2.DataSet(nodes, 2)), [(m0, m0, None)]))
+    with pytest.raises(op2.MapValueError):
+        bmat(op2.INC, (m2, m2))
+    bmat(op2.INC, (m0, m0))
